@@ -10,6 +10,7 @@ H2D/D2H inside the timed region.  `--impl reference` times the reference's own C
 cores of the same box.
 
     python bench.py --gpus 1 --steps 5 --warmup 3
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs /tmp/b200_outputs
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 5 --warmup 3
 """
@@ -237,6 +238,16 @@ def verify_against_oracle(bs, pairs, pcm_d, pcm_off, ratios, n_sample, seed):
                     "MaxScoreAligner) on a seeded sample; offsets exact, scores <= 1e-5 relative"}
 
 
+def dump_outputs(path, results):
+    """Write what the last timed step returned, one float64 .npy per array (int32 offsets and ratio
+    indices are exact in float64), so that two builds can be compared output for output.  The inputs
+    are seeded, so the same arguments give the same inputs on every run.  24 B per pair: even 8 GPUs x
+    512 pairs stay far below 64 MB, so nothing is sampled."""
+    os.makedirs(path, exist_ok=True)
+    for name, v in results.items():
+        np.save(os.path.join(path, name + ".npy"), v.cpu().numpy().astype(np.float64))
+
+
 def measured_traffic():
     """DRAM bytes per launch of the dominant kernel from this round's `ncu --set full` capture
     (profiles/r2_vad_traffic.json, written by tools/ncu_traffic.py from the .ncu-rep)."""
@@ -365,6 +376,13 @@ def run_gpu(args):
     elapsed_ms = distributed.max_over_ranks(local_ms, dev)
     launches = h.launch_count - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        if gather:   # the caller on rank 0 receives every rank's pairs: (score, offset, k) columns
+            last = state["last"]
+            dump_outputs(args.dump_outputs, {"best_score": last[:, 0], "best_offset": last[:, 1],
+                                             "best_k": last[:, 2]})
+        else:
+            dump_outputs(args.dump_outputs, out)
     per_rank = None
     if world > 1:  # every rank's own device time and SM clock, for the record
         mine = torch.tensor([local_ms / steps, float(clocks.get("sm_mhz") or 0.0),
@@ -655,7 +673,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ordered-calls", action="store_true",
                     help="timed steps call b2_sync_batch with B2_DEVICE instead of B2_DEVICE_RESIDENT (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the per-pair results of the last one (best_score, "
+                         "best_offset, best_k) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:
